@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 nearest-neighbour path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c3|c2|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c3|c2|c4|c5] [--dump-outputs DIR]
 
 Metric (BASELINE.json): Chamfer query-points/second on 2 x (1e6 x 3) fp32 uniform-random clouds
 (config "C3", SURVEY.md 8d): one step = one fused bidirectional Chamfer (+ Hausdorff statistics) of
@@ -24,6 +24,10 @@ one pair, grid build included; value = (n + m) * pairs / time.
   library on the launching stream (pcu_b200_workspace_set_profiling), algorithmic bytes per unit as
   in SURVEY.md 8d, peak = MEASURED_PEAKS.json hbm_gbs; `traffic` = ncu dram bytes of that kernel from
   the capture committed under profiles/ (profiles/dram_traffic.json).
+* `--dump-outputs DIR`: after the timed steps, rank 0 writes what the timed call returned in the last step to
+  DIR/<name>.npy (float32 / float64), so that two builds can be compared output for output on the same seeded
+  inputs: `chamfer` (C3), `chamfer_per_pair` + `chamfer_sum` (C5), `knn_dist` + `knn_idx` (C2 / C4; C4 as a fixed,
+  seeded sample of rows, listed in `rows`).
 * `cpu_baseline` / `--impl reference`: the reference's own nanoflann path (oracle/_ref, compiled from
   /root/reference/external/nanoflann in place) driven like point_cloud_utils.chamfer_distance (three
   tree builds per direction, OpenMP sweep, numpy norm/mean) on the box's host cores;
@@ -52,6 +56,7 @@ WORKLOADS = {
                batch=1024),
 }
 ALGO_BYTES_PER_QPT = {"c3": 24.0, "c2": 36.0, "c4": 205.2, "c5": 24.0}   # SURVEY.md 8(d)
+DUMP_BUDGET = 48 << 20   # --dump-outputs: bytes of sampled output rows (C4's 1.9 GB of results); row numbers come on top
 E2E_API = {
     "c3": "pcu.chamfer_distance(numpy, numpy) -> pcu_b200_chamfer_host_f32",
     "c2": "pcu.k_nearest_neighbors(numpy, numpy, 1) -> pcu_b200_knn_host_f32",
@@ -275,8 +280,32 @@ class Bench:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.SUM)
         return float(t.item())
 
+    def host_outputs(self, wl_key, result):
+        """What a caller of the timed call receives, as float32 / float64 numpy arrays (indices as float64, exact below
+        2^53).  Outputs larger than DUMP_BUDGET in all are cut to the same fixed, seeded sample of rows of each array;
+        the sampled row numbers are then returned as `rows`."""
+        torch = self.torch
+        if wl_key == "c3":
+            named = {"chamfer": result}
+        elif wl_key == "c5":
+            named = {"chamfer_per_pair": result[0], "chamfer_sum": result[1]}
+        else:
+            named = {"knn_dist": result[0], "knn_idx": result[1]}
+        total = sum(t.numel() * (4 if t.dtype == torch.float32 else 8) for t in named.values())
+        if total > DUMP_BUDGET:
+            n = next(iter(named.values())).shape[0]
+            rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BUDGET * n // total, replace=False))
+            sel = torch.from_numpy(rows).to(self.dev)
+            named = {name: t.index_select(0, sel) for name, t in named.items()}
+            named["rows"] = rows
+        out = {}
+        for name, t in named.items():
+            a = t.cpu().numpy() if isinstance(t, torch.Tensor) else t
+            out[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+        return out
+
     # -- device-resident arm of one workload: (value, ms_per_step, launches per step, stage_ms, units/step all ranks)
-    def device_arm(self, wl_key, xd, yd, local_batch, steps, warmup, sample_clocks):
+    def device_arm(self, wl_key, xd, yd, local_batch, steps, warmup, sample_clocks, keep_outputs=False):
         torch, pcu, bmod = self.torch, self.pcu, self.bmod
         wl = WORKLOADS[wl_key]
         n, m, k = wl["n"], wl["m"], wl["k"]
@@ -288,12 +317,11 @@ class Bench:
                     return bmod.distributed_chamfer_sum(xd, yd, exchange)
                 return pcu.chamfer_distance(xd, yd)                     # 0-dim CUDA tensor, no synchronisation
             if wl_key == "c5":
-                _, total = bmod.batched_chamfer(xd, yd, return_sum=True)   # fp64 sum of this rank's pairs
+                vals, total = bmod.batched_chamfer(xd, yd, return_sum=True)   # per pair, and the fp64 sum of this rank's pairs
                 if self.world > 1:
                     exchange.submit(total.reshape(1))
-                return total
-            pcu.k_nearest_neighbors(xd, yd, k)
-            return None
+                return vals, total
+            return pcu.k_nearest_neighbors(xd, yd, k)
 
         units_rank = ((n + m) if wl_key in ("c3", "c5") else n) * local_batch
         for _ in range(warmup):
@@ -311,13 +339,17 @@ class Bench:
         for s in range(steps):
             self.flush.fill_(s & 0xff)      # evict inputs / scratch from L2 (outside the interval)
             starts[s].record()
-            device_step()
+            result = device_step()
             if s == steps - 1:
                 exchange.wait()             # the last interval ends after the last collective
             stops[s].record()
+            if s < steps - 1:
+                result = None               # freed as each step ends; only the last step's results are kept
         self.barrier()
         launches = pcu.launch_count() - launches0
         clocks = sampler.stop() if sampler else None
+        outputs = self.host_outputs(wl_key, result) if keep_outputs else None
+        del result
         total_ms = self.reduce_max(sum(a.elapsed_time(b) for a, b in zip(starts, stops)))
         units = self.reduce_sum(units_rank)
         ms_per_step = total_ms / steps
@@ -337,7 +369,7 @@ class Bench:
                 stage_ms[key] = stage_ms.get(key, 0.0) + val / reps
         internal._set_profiling(self.local, self.stream, False)
         return dict(value=value, ms_per_step=ms_per_step, launches=launches, stage_ms=stage_ms, units=units,
-                    units_rank=units_rank, clocks=clocks)
+                    units_rank=units_rank, clocks=clocks, outputs=outputs)
 
     def place_host_buffers(self, xh, yh):
         """Page-locked copies of the two input clouds, placed on the NUMA node from which this GPU reads fastest.
@@ -451,7 +483,11 @@ def main():
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c5", action="store_true", help="skip the c5_strong object beside the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (rank 0, GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     wl_key = args.workload
     if args.impl == "reference":
@@ -473,7 +509,12 @@ def main():
     xd = torch.from_numpy(xh).to(dev)
     yd = torch.from_numpy(yh).to(dev)
 
-    res = B.device_arm(wl_key, xd, yd, local_batch, args.steps, args.warmup, sample_clocks=True)
+    dump = args.dump_outputs is not None and rank == 0
+    res = B.device_arm(wl_key, xd, yd, local_batch, args.steps, args.warmup, sample_clocks=True, keep_outputs=dump)
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in res["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     value, ms_per_step, stage_ms = res["value"], res["ms_per_step"], res["stage_ms"]
     peak, peak_src = measured_peak()
     algo_bytes = ALGO_BYTES_PER_QPT[wl_key] * res["units_rank"]

@@ -24,6 +24,7 @@ their conventions: ``(n,)`` squeeze for k == 1, int64 indices, ``ValueError`` fo
 Parity status: PINNED (see tests/test_oracle.py).
 """
 import ctypes
+import hashlib
 import os
 import subprocess
 
@@ -54,6 +55,12 @@ def build(quiet=True):
 
 def have_reference():
     return os.path.exists(_REF_PATH)
+
+
+def array_digest(a):
+    """SHA-256 of an array's dtype, shape and bytes: lets a golden file pin a large output exactly in 64 characters."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()
 
 
 def resolve_impl(impl=None):

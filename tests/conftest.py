@@ -21,7 +21,7 @@ def golden_names(prefix_exclude=("metrics_", "c1_metrics")):
 
 
 def knn_golden_names():
-    return [n for n in golden_names() if "metrics" not in n and not n.startswith(("morton", "sinkhorn"))]
+    return [n for n in golden_names() if "metrics" not in n and not n.startswith(("morton", "sinkhorn", "fresh"))]
 
 
 def metric_golden_names():
@@ -30,6 +30,14 @@ def metric_golden_names():
 
 def load_golden(name):
     return np.load(os.path.join(GOLDEN, name + ".npz"))
+
+
+def assert_pinned(oracle, g, key, got):
+    """`got` equals the array a fresh_* fixture pins under `key` (oracle/make_golden_fresh.py): first its sampled
+    rows, then, through the digest, every element."""
+    rows = g[key + "_rows"]
+    assert np.array_equal(got[rows], g[key + "_sample"]), key
+    assert oracle.array_digest(got) == str(g[key + "_digest"]), key
 
 
 def knn_cases(g):

@@ -1,12 +1,13 @@
 """64-bit Morton codes (SURVEY.md 8f, N3; /root/reference/src/morton.cpp, src/common/morton_code.cpp).
 Integer work: everything is compared bit for bit -- the C restatement and the CUDA kernels against golden vectors
-produced by the reference's own MortonCode64 class (oracle/make_golden_morton.py) and, where oracle/_ref is present,
-against that library on fresh inputs.  `morton_knn(sort_dist=True)`: the window is pinned; the order inside it is the
-intended one (by distance to the query), which the reference itself leaves undefined (uninitialised comparator state)."""
+produced by the reference's own MortonCode64 class (oracle/make_golden_morton.py) and against what that library
+returned on larger seeded inputs (oracle/make_golden_fresh.py).  `morton_knn(sort_dist=True)`: the window is pinned;
+the order inside it is the intended one (by distance to the query), which the reference itself leaves undefined
+(uninitialised comparator state)."""
 import numpy as np
 import pytest
 
-from conftest import load_golden
+from conftest import assert_pinned, load_golden
 
 
 def _check_against_golden(M, **kw):
@@ -36,19 +37,20 @@ def test_restatement_matches_reference_goldens(oracle):
 
 
 def test_restatement_matches_reference_library_on_fresh_inputs(oracle):
-    if not oracle.have_morton_reference():
-        pytest.skip("oracle/_ref/libpcu_ref_morton.so not built here")
+    """The reference library's outputs on these seeded inputs are stored in tests/golden/fresh_morton_ref.npz."""
+    g = load_golden("fresh_morton_ref")
     rng = np.random.default_rng(5)
     pts = rng.integers(-(1 << 20), 1 << 20, (50000, 3)).astype(np.int32)
     a = oracle.morton_encode(pts, impl="port")
-    assert np.array_equal(a, oracle.morton_encode(pts, impl="reference"))
+    assert_pinned(oracle, g, "encode_a", a)
     b = oracle.morton_encode(rng.integers(-(1 << 19), 1 << 19, (50000, 3)).astype(np.int32), impl="port")
-    for fn in (oracle.morton_add, oracle.morton_subtract):
-        assert np.array_equal(fn(a, b, impl="port"), fn(a, b, impl="reference"))
-    assert np.array_equal(oracle.morton_decode(a, impl="port"), oracle.morton_decode(a, impl="reference"))
+    assert_pinned(oracle, g, "encode_b", b)
+    assert_pinned(oracle, g, "add", oracle.morton_add(a, b, impl="port"))
+    assert_pinned(oracle, g, "subtract", oracle.morton_subtract(a, b, impl="port"))
+    assert_pinned(oracle, g, "decode", oracle.morton_decode(a, impl="port"))
     s = np.sort(a)
     for k in (1, 5, 64):
-        assert np.array_equal(oracle.morton_knn(s, b[:3000], k, False, impl="port"), oracle.morton_knn(s, b[:3000], k, False, impl="reference"))
+        assert_pinned(oracle, g, "knn_k%d" % k, oracle.morton_knn(s, b[:3000], k, False, impl="port"))
     # the arithmetic is the arithmetic of the encoded vectors (no overflow inside 21 bits)
     small = rng.integers(-1000, 1000, (1000, 3)).astype(np.int32)
     other = rng.integers(-1000, 1000, (1000, 3)).astype(np.int32)

@@ -1,10 +1,10 @@
 """CPU: the oracle (our restatement of the reference's kd-tree path) is pinned against the golden
-vectors generated from the reference's own nanoflann header (oracle/make_golden.py), and, where
-oracle/_ref is available, against that library directly on fresh inputs."""
+vectors generated from the reference's own nanoflann header (oracle/make_golden.py), and against
+what that library returned on larger seeded inputs (oracle/make_golden_fresh.py)."""
 import numpy as np
 import pytest
 
-from conftest import knn_cases, knn_golden_names, load_golden, metric_golden_names
+from conftest import assert_pinned, knn_cases, knn_golden_names, load_golden, metric_golden_names
 
 
 @pytest.mark.parametrize("name", knn_golden_names())
@@ -59,19 +59,23 @@ def test_conventions(oracle):
 
 
 def test_port_matches_reference_library_on_fresh_inputs(oracle):
-    if not oracle.have_reference():
-        pytest.skip("oracle/_ref not built here")
+    """The reference library's outputs on these seeded inputs are stored in tests/golden/fresh_knn_ref.npz."""
+    g = load_golden("fresh_knn_ref")
     rng = np.random.default_rng(11)
     for dt in (np.float32, np.float64):
+        sfx = np.dtype(dt).name
         q = rng.random((3000, 3)).astype(dt)
         d = np.concatenate([rng.random((4000, 3)), rng.random((500, 3)).round(1)]).astype(dt)
+        assert oracle.array_digest(q) == str(g[sfx + "_query_digest"]), "numpy generated other inputs than the golden's"
+        assert oracle.array_digest(d) == str(g[sfx + "_dataset_digest"]), "numpy generated other inputs than the golden's"
         for k, leaf in ((1, 10), (5, 3), (33, 10)):
             a = oracle.k_nearest_neighbors(q, d, k, max_points_per_leaf=leaf, impl="port")
-            b = oracle.k_nearest_neighbors(q, d, k, max_points_per_leaf=leaf, impl="reference")
-            assert np.array_equal(a[1], b[1]) and np.array_equal(a[0], b[0])
-    # the OpenMP path (n >= 100000) gives the same rows as the serial one
+            assert_pinned(oracle, g, "%s_k%d_leaf%d_idx" % (sfx, k, leaf), a[1])
+            assert_pinned(oracle, g, "%s_k%d_leaf%d_dist" % (sfx, k, leaf), a[0])
+    # the OpenMP path (n >= 100000) gives the same rows as the reference's serial one
     q = rng.random((100000, 3), dtype=np.float32)
     d = rng.random((20000, 3), dtype=np.float32)
+    assert oracle.array_digest(q) == str(g["serial_query_digest"]) and oracle.array_digest(d) == str(g["serial_dataset_digest"])
     a = oracle.k_nearest_neighbors(q, d, 2, num_threads=-1, impl="port")
-    b = oracle.k_nearest_neighbors(q, d, 2, num_threads=0, impl="reference")
-    assert np.array_equal(a[1], b[1]) and np.array_equal(a[0], b[0])
+    assert_pinned(oracle, g, "serial_k2_idx", a[1])
+    assert_pinned(oracle, g, "serial_k2_dist", a[0])
