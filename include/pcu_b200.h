@@ -329,6 +329,28 @@ int pcu_b200_voxel_downsample_f64(pcu_b200_workspace* ws, const double* points, 
                                   int min_points_per_voxel, double* out_points, void* out_attrib, int32_t* out_counts, int64_t* out_rows,
                                   void* stream);
 
+/* ---- Poisson-disk down-sampling ------------------------------------------------------------------
+ * Replaces downsample_point_cloud_poisson_disk (src/sample_point_cloud.cpp:240-333; exported at
+ * point_cloud_utils/__init__.py:4-5).  The reference's sampler (libigl's blue-noise loop, seeded through rand()) is not
+ * in its tree; the result here is defined instead as the greedy maximal independent set in ascending key order:
+ *   key(i) = (h(i) << 32) | i,  h(i) = mix32(seed ^ mix32(i * 0x9e3779b9 + 0x85ebca6b))  (mix32: normals.cuh);
+ *   rows i and j conflict iff d2(i, j) < r2, with the reference-rounded d2 of this library and r2 = (T)r * (T)r in the
+ *   cloud's precision T; a row is a sample iff it conflicts with no sample of smaller key.
+ * Unique (independent of scheduling), separated and maximal.  out_idx: int32 rows of the samples, ASCENDING (the
+ * reference returns its placement order); capacity n.  out_count: device int64.
+ * target_num_samples > 0: `radius` is ignored and the reference's radius search (:278-326: arange(n) when the target is
+ * >= n, halving from |bbox| / 50, doubling, at most 20 bisection steps with sample_num_tolerance) runs operation for
+ * operation in T; the call then synchronises `stream` once per radius trial (and once for the bounding box).  Without
+ * it nothing synchronises.  Argument errors (:265-270): target_num_samples <= 0 with radius <= 0, sample_num_tolerance
+ * outside (0, 1].  ABI version 3 is unchanged: the entries are an addition, detected by symbol.  DEVICE pointers. */
+int pcu_b200_poisson_disk_downsample_f32(pcu_b200_workspace* ws, const float* points, int64_t n, double radius, int target_num_samples,
+                                         uint32_t seed, float sample_num_tolerance, int32_t* out_idx, int64_t* out_count, void* stream);
+int pcu_b200_poisson_disk_downsample_f64(pcu_b200_workspace* ws, const double* points, int64_t n, double radius, int target_num_samples,
+                                         uint32_t seed, float sample_num_tolerance, int32_t* out_idx, int64_t* out_count, void* stream);
+/* The last Poisson-disk call on this workspace (synchronises the device): out[0] radius trials, out[1] rounds of the
+ * parallel MIS summed over its trials. */
+int pcu_b200_debug_poisson_stats(pcu_b200_workspace* ws, int64_t out[2]);
+
 /* ---- dense pairwise distances and Sinkhorn (SURVEY.md 8f, N4) -------------------------------
  * Replace the numpy code of point_cloud_utils/_sinkhorn.py: pairwise_distances (:4-34), sinkhorn (:37-126) and the
  * cost (P * M).sum() of earth_movers_distance (:129-156).  DEVICE pointers, row-major dense arrays:
@@ -400,6 +422,11 @@ int pcu_b200_voxel_downsample_host_f32(pcu_b200_workspace* ws, const float* poin
 int pcu_b200_voxel_downsample_host_f64(pcu_b200_workspace* ws, const double* points, int64_t n, const void* attrib, int attrib_cols,
                                        int attrib_is_f64, const double voxel_size[3], const double min_bound[3], const double max_bound[3],
                                        int min_points_per_voxel, double* out_points, void* out_attrib, int32_t* out_counts, int64_t* out_rows);
+/* Poisson-disk down-sampling on HOST arrays: out_idx (capacity n) and out_count are HOST memory */
+int pcu_b200_poisson_disk_downsample_host_f32(pcu_b200_workspace* ws, const float* points, int64_t n, double radius, int target_num_samples,
+                                              uint32_t seed, float sample_num_tolerance, int32_t* out_idx, int64_t* out_count);
+int pcu_b200_poisson_disk_downsample_host_f64(pcu_b200_workspace* ws, const double* points, int64_t n, double radius, int target_num_samples,
+                                              uint32_t seed, float sample_num_tolerance, int32_t* out_idx, int64_t* out_count);
 int pcu_b200_deduplicate_host_f32(pcu_b200_workspace* ws, const float* points, int64_t n, double epsilon, const void* faces, int64_t n_faces,
                                   int face_cols, int faces_are_i64, float* out_points, int32_t* out_svi, int32_t* out_svj, void* out_faces,
                                   int64_t* out_counts);

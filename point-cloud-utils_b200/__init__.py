@@ -39,7 +39,8 @@ except ImportError as _e:  # pragma: no cover - exercised only on a broken insta
 __all__ = ["k_nearest_neighbors", "one_sided_hausdorff_distance", "hausdorff_distance", "chamfer_distance",
            "batched_chamfer_distance", "estimate_point_cloud_normals_knn", "estimate_point_cloud_normals_ball",
            "morton_encode", "morton_decode", "morton_add", "morton_subtract", "morton_knn", "pairwise_distances", "sinkhorn",
-           "earth_movers_distance", "downsample_point_cloud_on_voxel_grid", "deduplicate_point_cloud",
+           "earth_movers_distance", "downsample_point_cloud_on_voxel_grid", "downsample_point_cloud_poisson_disk",
+           "deduplicate_point_cloud",
            "deduplicate_mesh_vertices", "prepare_cloud", "pinned_empty", "PreparedCloud", "device_count",
            "current_device", "launch_count"]
 
@@ -885,6 +886,65 @@ def downsample_point_cloud_on_voxel_grid(voxel_size, points, *args, min_bound=No
         _, ret_ai = _voxel_internal(points, attribs[i], voxel_size, min_bound, max_bound, min_points_per_voxel, device)
         ret.append(ret_ai)
     return tuple(ret) if len(ret) > 1 else ret_v
+
+
+def downsample_point_cloud_poisson_disk(v, radius, target_num_samples=-1, random_seed=0, sample_num_tolerance=0.04, *, device=None):
+    """
+    Downsample a point set so that samples are approximately evenly spaced.
+
+    Args:
+        v : an (n, 3)-shaped float32 / float64 array (or tensor) of points
+        radius : desired separation between points (ignored when target_num_samples > 0)
+        target_num_samples : if positive, search for the radius whose sample count lies within sample_num_tolerance of it
+        random_seed : 32-bit seed of the sample priorities; 0 draws one from NumPy's global RNG (so np.random.seed makes
+                      the call reproducible)
+        sample_num_tolerance : relative tolerance of target_num_samples, in (0, 1]
+        device : see `k_nearest_neighbors` (keyword only).
+
+    Returns:
+        p_idx : an (m,)-shaped int32 array of row indices into v, ASCENDING (numpy for numpy input, an int32 CUDA tensor
+                on v's device for a CUDA tensor)
+
+    Mirrors the reference's point_cloud_utils/__init__.py:4-5 and src/sample_point_cloud.cpp:240-333:
+    name, arguments, defaults, argument errors and the target_num_samples search (run in v's precision).  The samples
+    themselves are the greedy maximal independent set in the order of a seeded hash of the row: rows i and j conflict
+    when their squared distance, rounded in v's precision like every distance of this library, is below radius * radius
+    (also rounded in v's precision); visiting the rows by priority, a row is kept when it conflicts with no row kept
+    before it.  No two samples conflict and every other row conflicts with a sample.  The reference's sampler (libigl's
+    blue-noise loop) draws its priorities from rand() and returns the samples in placement order; neither is
+    reproducible, so its exact output is not.
+    """
+    if target_num_samples <= 0 and radius <= 0.0:                               # :265-267
+        raise ValueError("Cannot have both num_samples <= 0 and radius <= 0")
+    tol = float(_np.float32(sample_num_tolerance))                               # the binding takes a float
+    if tol > 1.0 or tol <= 0.0:                                                  # :268-270
+        raise ValueError("sample_num_tolerance must be in (0, 1]")
+    if not (0 <= int(random_seed) < 2 ** 32):
+        raise ValueError("random_seed must fit in 32 unsigned bits (got %d)" % int(random_seed))
+    if not (-2 ** 31 <= int(target_num_samples) < 2 ** 31):
+        raise ValueError("target_num_samples must fit in a 32-bit int (got %d)" % int(target_num_samples))
+    seed = int(random_seed) if int(random_seed) != 0 else int(_np.random.randint(1, 2 ** 32, dtype=_np.uint64))
+    if _is_tensor(v):
+        torch = _torch()
+        if v.dtype not in (torch.float32, torch.float64):
+            raise ValueError("Invalid scalar type (%s) for argument 'v'. Expected one of ['float32', 'float64']." % v.dtype)
+        if v.dim() != 2 or v.shape[-1] != 3 or v.shape[0] == 0:
+            raise ValueError("v must have shape (n, 3) with n > 0, got " + str(tuple(v.shape)))
+        pts = v.detach().contiguous()
+        if not pts.is_cuda:
+            return torch.from_numpy(downsample_point_cloud_poisson_disk(pts.numpy(), radius, target_num_samples, seed,
+                                                                        sample_num_tolerance, device=device))
+        _same_device(pts, device)
+        n = pts.shape[0]
+        idx = torch.empty(n, dtype=torch.int32, device=pts.device)
+        count = torch.empty(1, dtype=torch.int64, device=pts.device)
+        _pcu_internal._poisson_device(pts.dtype == torch.float64, pts.data_ptr(), n, float(radius), int(target_num_samples), seed,
+                                      tol, idx.data_ptr(), count.data_ptr(), pts.device.index or 0, _stream_of(pts))
+        return idx[:int(count.item())]
+    if type(v) != _np.ndarray:
+        raise ValueError("Invalid type for v, must be a NumPy array, but got " + str(type(v)) + ".")
+    return _pcu_internal.downsample_point_cloud_poisson_disk_internal(v, float(radius), int(target_num_samples), seed, tol,
+                                                                      _dev(device))
 
 
 def batched_chamfer_distance(x, y, max_points_per_leaf=10, *, device=None):

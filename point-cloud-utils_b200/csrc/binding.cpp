@@ -804,6 +804,50 @@ void deduplicate_device(bool is_f64, uintptr_t pts, int64_t n, double epsilon, u
     check(status);
 }
 
+// ---- Poisson-disk down-sampling (src/sample_point_cloud.cpp:240-333): numpy in, int32 rows out ----
+template <typename T>
+py::array_t<int32_t> poisson_numpy(const py::array& v_in, double radius, int target, uint32_t seed, float tol, int device) {
+    auto pts = dense<T>(v_in);
+    const int64_t n = pts.shape(0);
+    py::array_t<int32_t> idx({(py::ssize_t)n});
+    int64_t kept = 0;
+    Slot& slot = pool().get(device, kHostKey);
+    int status;
+    {
+        CallScope scope(slot);
+        status = sizeof(T) == 4 ? pcu_b200_poisson_disk_downsample_host_f32(slot.ws, (const float*)pts.data(), n, radius, target, seed, tol,
+                                                                            idx.mutable_data(), &kept)
+                                : pcu_b200_poisson_disk_downsample_host_f64(slot.ws, (const double*)pts.data(), n, radius, target, seed, tol,
+                                                                            idx.mutable_data(), &kept);
+    }
+    check(status);
+    idx.resize({(py::ssize_t)kept});
+    return idx;
+}
+
+py::array downsample_point_cloud_poisson_disk_internal(const py::array& v, double radius, int target_num_samples, uint32_t random_seed,
+                                                       float sample_num_tolerance, int device) {
+    check_shapes(v, v, "v", "v");
+    const Dt dt = common_dtype(v, v, "v", "v");
+    const int dev = current_device_or_default(device);
+    return dt == Dt::f32 ? (py::array)poisson_numpy<float>(v, radius, target_num_samples, random_seed, sample_num_tolerance, dev)
+                         : (py::array)poisson_numpy<double>(v, radius, target_num_samples, random_seed, sample_num_tolerance, dev);
+}
+
+void poisson_device(bool is_f64, uintptr_t pts, int64_t n, double radius, int target, uint32_t seed, float tol, uintptr_t out_idx,
+                    uintptr_t out_count, int device, uintptr_t stream) {
+    Slot& slot = pool().get(device, stream);
+    int status;
+    {
+        CallScope scope(slot);
+        status = is_f64 ? pcu_b200_poisson_disk_downsample_f64(slot.ws, (const double*)pts, n, radius, target, seed, tol, (int32_t*)out_idx,
+                                                               (int64_t*)out_count, (void*)stream)
+                        : pcu_b200_poisson_disk_downsample_f32(slot.ws, (const float*)pts, n, radius, target, seed, tol, (int32_t*)out_idx,
+                                                               (int64_t*)out_count, (void*)stream);
+    }
+    check(status);
+}
+
 // ---- dense pairwise distances / Sinkhorn on device pointers (the Python layer owns the arrays) ----
 void pairwise_device(bool is_f64, uintptr_t a, uintptr_t b, int64_t nb, int64_t n, int64_t m, int d, int norm_kind, double p,
                      uintptr_t out, int device, uintptr_t stream) {
@@ -1003,6 +1047,16 @@ PYBIND11_MODULE(_pcu_internal, mod) {
     mod.def("_stats_prepared_device", &stats_prepared_device);
     mod.def("_voxel_downsample_device", &voxel_downsample_device);
     mod.def("_deduplicate_device", &deduplicate_device);
+    mod.def("downsample_point_cloud_poisson_disk_internal", &downsample_point_cloud_poisson_disk_internal, py::arg("v"), py::arg("radius"),
+            py::arg("target_num_samples"), py::arg("random_seed"), py::arg("sample_num_tolerance"), py::arg("device") = -1);
+    mod.def("_poisson_device", &poisson_device);
+    // (radius trials, MIS rounds) of the last Poisson-disk call on the workspace of (device, stream); stream None = numpy path
+    mod.def("_poisson_stats", [](int device, py::object stream) {
+        Slot& slot = pool().get(current_device_or_default(device), stream.is_none() ? kHostKey : stream.cast<uintptr_t>());
+        int64_t out[2] = {0, 0};
+        { CallScope scope(slot); check(pcu_b200_debug_poisson_stats(slot.ws, out)); }
+        return py::make_tuple(out[0], out[1]);
+    }, py::arg("device") = -1, py::arg("stream") = py::none());
     mod.def("_pairwise_device", &pairwise_device);
     mod.def("_sinkhorn_device", &sinkhorn_device);
     mod.def("morton_encode", &morton_encode, py::arg("pts"), py::arg("num_threads") = -1, py::arg("device") = -1,

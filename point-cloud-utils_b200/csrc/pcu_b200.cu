@@ -31,6 +31,7 @@
 #include "sinkhorn.cuh"
 #include "voxel.cuh"
 #include "dedup.cuh"
+#include "poisson.cuh"
 
 using namespace pcu;
 
@@ -221,6 +222,8 @@ struct pcu_b200_workspace {
     int marks_used = 0;
     bool host_marks = false;      // marks 9 and 10 belong to the last call
     HostStager* stager = nullptr; // pinned ring + copy threads for pageable inputs of the host entry points (created on first use)
+    long long poisson_trials = 0;                  // radius trials of the last Poisson-disk call
+    unsigned long long* poisson_rounds = nullptr;  // device: MIS rounds of the last Poisson-disk call, summed over its trials
 };
 
 // A cloud binned once (pcu_b200_cloud_prepare_*): its cell-sorted points, cell table, grid header, wall tables and
@@ -1159,6 +1162,166 @@ int voxel_downsample_dispatch(pcu_b200_workspace* ws, const T* pts, long long n,
                                              (float*)out_attr, out_counts, out_rows, stream);
 }
 
+// ---- Poisson-disk down-sampling (downsample_point_cloud_poisson_disk, src/sample_point_cloud.cpp:240-333) -------
+template <typename T> T unordered_host(typename std::conditional<sizeof(T) == 4, uint32_t, unsigned long long>::type u) {
+    using B = decltype(u);
+    const B sign = (B)1 << (8 * sizeof(B) - 1);
+    const B bits = (u & sign) ? (u & ~sign) : ~u;
+    T v;
+    std::memcpy(&v, &bits, sizeof v);
+    return v;
+}
+
+// One call: the key sort and the gather into key order once, then one radius trial per value of r the target search
+// asks for (a single trial without target_num_samples).  A trial enqueues binning -> cell order -> the cooperative MIS
+// launch -> flags -> compaction into out_idx / out_count; the target search reads each trial's count back (one stream
+// synchronisation per trial, plus one for the bounding box), the radius form does not synchronise at all.
+int poisson_check_args(const pcu_b200_workspace* ws, const void* pts, long long n, double radius, int target, float tol,
+                       const void* out_idx, const void* out_count) {
+    if (!ws) return fail(PCU_B200_INVALID_ARGUMENT, "null workspace");
+    // the checks of the binding (:265-270), then the shape rules of this library
+    if (target <= 0 && radius <= 0.0) return fail(PCU_B200_INVALID_ARGUMENT, "Cannot have both num_samples <= 0 and radius <= 0");
+    if (tol > 1.0 || tol <= 0.0) return fail(PCU_B200_INVALID_ARGUMENT, "sample_num_tolerance must be in (0, 1]");
+    if (!pts || n <= 0) return fail(PCU_B200_INVALID_ARGUMENT, "points must be a non-empty (n, 3) array");
+    if (n >= 0x7fffffffLL) return fail(PCU_B200_INVALID_ARGUMENT, "point cloud too large (%lld rows; at most 2^31 - 2 are supported)", n);
+    if (!out_idx || !out_count) return fail(PCU_B200_INVALID_ARGUMENT, "null output pointer");
+    return PCU_B200_OK;
+}
+
+template <typename T>
+int poisson_device(pcu_b200_workspace* ws, const T* pts, long long n, double radius, int target, unsigned seed, float tol,
+                   int* out_idx, long long* out_count, cudaStream_t stream) {
+    using bits_t = typename Real<T>::bits_t;
+    PCU_TRY(poisson_check_args(ws, pts, n, radius, target, tol, out_idx, out_count));
+    PCU_ON_DEVICE(ws);
+    PCU_TRY(adopt_stream(ws, stream));
+    ws->poisson_trials = 0;
+    if (!ws->poisson_rounds) PCU_CUDA(cudaMalloc((void**)&ws->poisson_rounds, sizeof(unsigned long long)));
+    PCU_CUDA(cudaMemsetAsync(ws->poisson_rounds, 0, sizeof(unsigned long long), stream));
+    const long long nblocks = (n + kThreads - 1) / kThreads;
+    if (target > 0 && (long long)target >= n) {            // :279-283
+        PCU_LAUNCH(poisson_all_rows_kernel, (unsigned)nblocks, kThreads, stream, n, out_idx, out_count);
+        return PCU_B200_OK;
+    }
+    const unsigned ntiles = (unsigned)((n + kSortTile - 1) / kSortTile);
+    struct Scratch { PoissonRec *a, *b; unsigned* hist; unsigned long long* totals; unsigned* base; int* constant; T* ranked; int* row_of;
+                     unsigned char* state; unsigned char* keep; unsigned* counts; unsigned* counters; bits_t* box; } sc;
+    auto carve = [&](Carver& cv) {
+        sc.a = cv.take<PoissonRec>((size_t)n);
+        sc.b = cv.take<PoissonRec>((size_t)n);
+        sc.hist = cv.take<unsigned>((size_t)kSortBins * ntiles);
+        sc.totals = cv.take<unsigned long long>(kSortBins);
+        sc.base = cv.take<unsigned>(kSortBins);
+        sc.constant = cv.take<int>(1);
+        sc.ranked = cv.take<T>((size_t)3 * n);
+        sc.row_of = cv.take<int>((size_t)n);
+        sc.state = cv.take<unsigned char>((size_t)n);
+        sc.keep = cv.take<unsigned char>((size_t)n);
+        sc.counts = cv.take<unsigned>((size_t)nblocks);
+        sc.counters = cv.take<unsigned>(5);           // 3 round counts + the grid barrier (poisson_mis_kernel)
+        sc.box = cv.take<bits_t>(6);
+    };
+    Carver measure(nullptr);
+    carve(measure);
+    PCU_TRY(grow_block(ws->aux, ws->aux_bytes, measure.off, stream, "Poisson-disk scratch"));
+    Carver cv(ws->aux);
+    carve(cv);
+    // the binned copy: the ranked points with a one-point dummy second cloud that is never binned (as normals_ball_device)
+    PlanSpec<T> spec;
+    spec.a = sc.ranked; spec.n = n; spec.b = sc.ranked; spec.m = 1;
+    spec.nsweeps = 1; spec.k = 1;
+    spec.occupancy = 0.125f;          // the cell budget; the cell size itself is held up by min_cell
+    spec.binning = 1;
+    spec.prepared_second = true;
+    Plan<T> plan;
+    plan.layout(nullptr, spec);
+    PCU_TRY(ensure_arena(ws, plan.total, stream));
+    plan.layout(ws->arena, spec);
+    plan.cv.v[0].hint_out = nullptr;
+
+    PCU_LAUNCH(poisson_keys_kernel, (unsigned)nblocks, kThreads, stream, n, seed, sc.a);
+    PoissonRec* sorted = nullptr;
+    PCU_TRY(radix_sort_records<PoissonRec>(sc.a, sc.b, n, 1, sc.hist, sc.totals, sc.base, sc.constant, stream, &sorted));
+    PCU_LAUNCH((poisson_gather_kernel<T>), (unsigned)nblocks, kThreads, stream, (const PoissonRec*)sorted, n, pts, sc.ranked, sc.row_of);
+
+    int mis_blocks = 0;
+    {
+        int sms = 0, fit = 0;
+        PCU_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ws->device));
+        PCU_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, poisson_mis_kernel<T>, kThreads, 0));
+        mis_blocks = (int)std::max<long long>(1, std::min<long long>(nblocks, (long long)std::max(1, fit) * sms));
+    }
+    auto trial = [&](T r) -> int {
+        ++ws->poisson_trials;
+        const T r2 = r * r;                                 // rr = r * r on a Scalar r (:72)
+        if (!(r2 > (T)0)) {                                 // nothing conflicts (also a NaN radius)
+            PCU_LAUNCH(poisson_all_rows_kernel, (unsigned)nblocks, kThreads, stream, n, out_idx, out_count);
+            return PCU_B200_OK;
+        }
+        plan.cv.v[0].min_cell = (float)std::min(1e30, 0.5 * std::sqrt((double)r2));
+        PCU_TRY(enqueue_binning(ws, plan, stream, nullptr, true));
+        PCU_LAUNCH((cell_order_kernel<T>), (unsigned)std::min<long long>(((long long)plan.cv.v[0].cell_cap + kThreads - 1) / kThreads, 148 * 64),
+                   kThreads, stream, plan.cv.v[0]);
+        PCU_CUDA(cudaMemsetAsync(sc.state, 0, (size_t)n, stream));
+        PCU_CUDA(cudaMemsetAsync(sc.counters, 0, 5 * sizeof(unsigned), stream));
+        Cloud<T> cl = plan.cv.v[0];
+        T rr = r2;
+        unsigned long long* rounds = ws->poisson_rounds;
+        void* args[] = {(void*)&cl, (void*)&rr, (void*)&sc.state, (void*)&sc.counters, (void*)&rounds};
+        PCU_CUDA(cudaLaunchCooperativeKernel((void*)poisson_mis_kernel<T>, dim3(mis_blocks), dim3(kThreads), args, 0, stream));
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        PCU_LAUNCH(poisson_flag_kernel, (unsigned)nblocks, kThreads, stream, (const unsigned char*)sc.state, (const int*)sc.row_of, n, sc.keep);
+        PCU_LAUNCH(keep_count_kernel, (unsigned)nblocks, kThreads, stream, (const unsigned char*)sc.keep, n, sc.counts);
+        PCU_LAUNCH(keep_offsets_kernel, 1, 1024, stream, sc.counts, nblocks, out_count);
+        PCU_LAUNCH(poisson_scatter_kernel, (unsigned)nblocks, kThreads, stream, (const unsigned char*)sc.keep, n, (const unsigned*)sc.counts, out_idx);
+        return PCU_B200_OK;
+    };
+    if (target <= 0) return trial((T)radius);
+
+    // target_num_samples > 0: the search of :285-326, operation for operation in the cloud's precision; every trial's
+    // sample count is read back before the next radius is chosen
+    long long* host_count = reinterpret_cast<long long*>(ws->host_slot);
+    auto run = [&](T r, long long& count) -> int {
+        PCU_TRY(trial(r));
+        PCU_CUDA(cudaMemcpyAsync(host_count, out_count, sizeof(long long), cudaMemcpyDeviceToHost, stream));
+        PCU_CUDA(cudaStreamSynchronize(stream));
+        count = *host_count;
+        return PCU_B200_OK;
+    };
+    const unsigned long long num_min = (unsigned long long)(int)((T)target * (T)(1.0f - tol));
+    const unsigned long long num_max = (unsigned long long)(int)((T)target * (T)(1.0f + tol));
+    PCU_CUDA(cudaMemsetAsync(sc.box, 0xff, 3 * sizeof(bits_t), stream));
+    PCU_CUDA(cudaMemsetAsync(sc.box + 3, 0, 3 * sizeof(bits_t), stream));
+    PCU_LAUNCH((poisson_bbox_kernel<T>), (unsigned)std::min<long long>(nblocks, 4 * 148), kThreads, stream, pts, n, sc.box);
+    bits_t* host_box = reinterpret_cast<bits_t*>(ws->host_slot + 64);
+    PCU_CUDA(cudaMemcpyAsync(host_box, sc.box, 6 * sizeof(bits_t), cudaMemcpyDeviceToHost, stream));
+    PCU_CUDA(cudaStreamSynchronize(stream));
+    T ext[3];
+    for (int a = 0; a < 3; ++a) ext[a] = unordered_host<T>(host_box[3 + a]) - unordered_host<T>(host_box[a]);
+    const T sq01 = ext[0] * ext[0] + ext[1] * ext[1];
+    const T bbsize = std::sqrt(sq01 + ext[2] * ext[2]);    // (bmax - bmin).norm()
+    T rmin = (T)((double)bbsize / 50.0), rmax = (T)((double)bbsize / 50.0);
+    long long count = 0;
+    do {
+        rmin = (T)((double)rmin / 2.0);
+        PCU_TRY(run(rmin, count));
+    } while ((unsigned long long)count < (unsigned long long)target);
+    // (the reference never ends this loop when bbsize is 0 or not finite -- the radius cannot grow: stop there)
+    do {
+        rmax = (T)((double)rmax * 2.0);
+        PCU_TRY(run(rmax, count));
+    } while ((unsigned long long)count > (unsigned long long)target && (T)((double)rmax * 2.0) > rmax);
+    int iter = 0;
+    while (iter < 20 && ((unsigned long long)count < num_min || (unsigned long long)count > num_max)) {
+        iter += 1;
+        const T cur = (T)((double)(T)(rmin + rmax) / 2.0);
+        PCU_TRY(run(cur, count));
+        if (count > (long long)target) rmin = cur;
+        if (count < (long long)target) rmax = cur;
+    }
+    return PCU_B200_OK;
+}
+
 // ---- dense pairwise distances, Sinkhorn (SURVEY.md 8f N4) ------------------------------------------------
 template <typename T>
 int pairwise_device(pcu_b200_workspace* ws, const T* a, const T* b, long long nb, long long n, long long m, int d, int norm_kind,
@@ -1376,6 +1539,7 @@ int pcu_b200_workspace_destroy(pcu_b200_workspace* ws) {
     if (ws->arena) cudaFree(ws->arena);
     if (ws->io) cudaFree(ws->io);
     if (ws->aux) cudaFree(ws->aux);
+    if (ws->poisson_rounds) cudaFree(ws->poisson_rounds);
     if (ws->handover) cudaEventDestroy(ws->handover);
     if (ws->hint_host) cudaFreeHost((void*)ws->hint_host);
     if (ws->own_stream) cudaStreamDestroy(ws->own_stream);
@@ -1552,6 +1716,29 @@ int pcu_b200_voxel_downsample_f64(pcu_b200_workspace* ws, const double* points, 
                                   void* stream) {
     return voxel_downsample_dispatch<double>(ws, points, n, attrib, attrib_cols, attrib_is_f64, voxel_size, min_bound, max_bound,
                                              min_points_per_voxel, out_points, out_attrib, out_counts, (long long*)out_rows, (cudaStream_t)stream);
+}
+
+int pcu_b200_poisson_disk_downsample_f32(pcu_b200_workspace* ws, const float* points, int64_t n, double radius, int target_num_samples,
+                                         uint32_t seed, float sample_num_tolerance, int32_t* out_idx, int64_t* out_count, void* stream) {
+    return poisson_device<float>(ws, points, n, radius, target_num_samples, seed, sample_num_tolerance, out_idx, (long long*)out_count,
+                                 (cudaStream_t)stream);
+}
+int pcu_b200_poisson_disk_downsample_f64(pcu_b200_workspace* ws, const double* points, int64_t n, double radius, int target_num_samples,
+                                         uint32_t seed, float sample_num_tolerance, int32_t* out_idx, int64_t* out_count, void* stream) {
+    return poisson_device<double>(ws, points, n, radius, target_num_samples, seed, sample_num_tolerance, out_idx, (long long*)out_count,
+                                  (cudaStream_t)stream);
+}
+int pcu_b200_debug_poisson_stats(pcu_b200_workspace* ws, int64_t out[2]) {
+    if (!ws || !out) return fail(PCU_B200_INVALID_ARGUMENT, "null argument");
+    PCU_ON_DEVICE(ws);
+    unsigned long long rounds = 0;
+    if (ws->poisson_rounds) {
+        PCU_CUDA(cudaDeviceSynchronize());
+        PCU_CUDA(cudaMemcpy(&rounds, ws->poisson_rounds, sizeof rounds, cudaMemcpyDeviceToHost));
+    }
+    out[0] = ws->poisson_trials;
+    out[1] = (int64_t)rounds;
+    return PCU_B200_OK;
 }
 
 int pcu_b200_pairwise_distances_f32(pcu_b200_workspace* ws, const float* a, const float* b, int64_t nb, int64_t n, int64_t m, int d,

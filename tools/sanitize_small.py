@@ -46,6 +46,8 @@ step("normals knn", lambda: pcu.estimate_point_cloud_normals_knn(v.astype(np.flo
 step("normals ball", lambda: pcu.estimate_point_cloud_normals_ball(v.astype(np.float32), 0.01, v.astype(np.float32), np.deg2rad(30), 5, weight_function="rbf"))
 step("normals ball, capped, fp64", lambda: pcu.estimate_point_cloud_normals_ball(v, 0.01, max_pts_per_ball=6))
 step("voxel down-sampling", lambda: pcu.downsample_point_cloud_on_voxel_grid(0.05, x, x.astype(np.float64)))
+step("poisson-disk down-sampling, radius and target", lambda: (pcu.downsample_point_cloud_poisson_disk(x, 0.05, random_seed=3),
+                                                               pcu.downsample_point_cloud_poisson_disk(v, 0., target_num_samples=300, random_seed=3)))
 step("deduplicate points", lambda: pcu.deduplicate_point_cloud(np.concatenate([x, x[:500]]), 1e-6))
 step("deduplicate mesh fp64", lambda: pcu.deduplicate_mesh_vertices(np.concatenate([x, x[:500]]).astype(np.float64), rng.integers(0, n, (3000, 3)).astype(np.int64), 0.0))
 pts_i = rng.integers(-1000, 1000, (n, 3)).astype(np.int32)
